@@ -214,6 +214,54 @@ def algorithmic_cost(N, S, side, R, B):
         lbs_bytes=N * (96 + 12 + 32 + 4) + B * N * 36)
 
 
+def dump_outputs(out_dir: str, model, loss) -> None:
+    """What a caller of the train step holds after it, as float32 `<name>.npy` files in `out_dir`: the loss, the feature net's
+    parameters, gradients and BatchNorm running statistics (each concatenated in the reference's order, so the files do not depend
+    on how a build packs its buffers) and geo_feature with its gradient.  About 12 MB at every config."""
+    import numpy as np
+    import torch
+    net = model.net
+
+    def cat(ts):
+        return torch.cat([t.reshape(-1) for t in ts])
+
+    arrays = {"loss": loss.detach(),
+              "net_params": cat(net.reference_tensors_from_flat(net.flat.detach())),
+              "net_grads": cat(net.reference_tensors_from_flat(net.flat.grad)),
+              "net_bn_running": cat([v for k, v in net.state_dict().items() if ".running_" in k]),
+              "geo_feature": model.geo_feature.detach(),
+              "geo_feature_grad": model.geo_feature.grad}
+    arrays = {k: v.float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, f"--dump-outputs: {total} bytes, more than 64 MB"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
+def model_state(model) -> dict:
+    """Copies of everything a training step changes: parameters, BatchNorm running statistics, Adam's moments and step counts, the
+    learning-rate schedule (load_model_state puts them back)."""
+    import torch
+    return dict(tensors=[t.detach().clone() for t in (model.net.flat, model.geo_feature, model.net.bn_running)],
+                adam={p: {k: v.clone() if torch.is_tensor(v) else v for k, v in st.items()} for p, st in model.optimizer.state.items()},
+                sched=model.scheduler.state_dict(), lrs=[g["lr"] for g in model.optimizer.param_groups])
+
+
+def load_model_state(model, saved) -> None:
+    """Back to `saved` (model_state); tensors in place, so the captured step graphs keep pointing at the live ones."""
+    import torch
+    with torch.no_grad():
+        for t, s in zip((model.net.flat, model.geo_feature, model.net.bn_running), saved["tensors"]):
+            t.copy_(s)
+    model.optimizer.state.clear()
+    for p, st in saved["adam"].items():
+        model.optimizer.state[p] = {k: v.clone() if torch.is_tensor(v) else v for k, v in st.items()}
+    model.scheduler.load_state_dict(saved["sched"])
+    for g, lr in zip(model.optimizer.param_groups, saved["lrs"]):
+        g["lr"] = lr
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -225,6 +273,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the config-4 (1 frame/GPU) and config-5 (novel-pose) side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="start the last timed step from the seeded model and optimizer state (so its "
+                    "inputs are identical from run to run) and write what it computed (loss, updated parameters, gradients) as "
+                    "DIR/<name>.npy, for output-for-output comparison of two builds")
     args = ap.parse_args()
     args.warmup = max(3, args.warmup) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
@@ -255,6 +306,7 @@ def main():
     wl = Stage1Workload(args.config, B, device=dev)
     wl.make_ground_truth()
     trainer = Stage1Trainer(wl.model, fused_adam=True)
+    seeded = model_state(wl.model) if args.dump_outputs else None      # before the first step
     iteration0 = 5000      # >= 1000: no scale ramp (SURVEY.md §8d)
 
     def barrier():
@@ -275,6 +327,8 @@ def main():
         for b in dev_batches.values():
             b["original_image"] = b["original_image"].clone()
 
+    last_loss = [None]        # of the latest step, detached: holding an eager step's graph would keep it alive into the next step
+
     def run_value(n, start):
         t0 = time.perf_counter()
         trainer.host_wait_s = trainer.host_enqueue_s = 0.0
@@ -283,7 +337,7 @@ def main():
             batch = dev_batches[tuple(wl.frame_ids(start + i, rank, world))]
             if _sleep_ms:
                 time.sleep(_sleep_ms * 1e-3)
-            trainer.step(batch, iteration0 + start + i, epoch=1)
+            last_loss[0] = trainer.step(batch, iteration0 + start + i, epoch=1).detach()
             if diag_ev is not None:
                 e = torch.cuda.Event(enable_timing=True); e.record(); diag_ev.append(e)
         if os.environ.get("GA_BENCH_DIAG") == "1" and rank == 0 and n > 2:
@@ -387,10 +441,27 @@ def main():
     run_value(args.warmup, 0)
     clocks.rows.clear()                    # keep only samples taken during the timed region
     l0 = _lib.launch_count() + trainer.replayed_launches
-    ms_value = timed(run_value, args.steps, args.warmup)
+    if args.dump_outputs:
+        # the last timed step starts from the seeded state, so that its inputs are identical from run to run (every step before it
+        # leaves a state that float-atomic summation order makes differ between runs): the steps before it are one timed window, the
+        # model and optimizer are put back untimed, and the last step is a second window
+        ms_value = timed(run_value, args.steps - 1, args.warmup)
+        trainer.finish()
+        trained = model_state(wl.model)
+        load_model_state(wl.model, seeded)
+        ms_value += timed(run_value, 1, args.warmup + args.steps - 1)
+    else:
+        ms_value = timed(run_value, args.steps, args.warmup)
     launches = _lib.launch_count() + trainer.replayed_launches - l0      # eager launches + the kernels inside the replayed step graphs
     clk = clocks.stop() if rank == 0 else {}
     fps = world * B * args.steps / (ms_value * 1e-3)
+    if args.dump_outputs:
+        # the timed trainer's own last step, settled (re-run if its binning buffer overflowed), before anything else moves the model
+        rerun = trainer.finish()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, wl.model, last_loss[0] if rerun is None else rerun)
+        load_model_state(wl.model, trained)    # the measurements below continue from the state the timed steps before it reached
+        del rerun, trained, seeded
 
     # ---- end to end through the public API with host batches ----------------------------------------------------------
     e2e = None

@@ -169,13 +169,15 @@ class Stage1Trainer:
         return out
 
     def finish(self):
-        """Settle the last step (re-run it if its binning buffer overflowed)."""
+        """Settle the last step (re-run it if its binning buffer overflowed).  Returns the loss of the re-run, None if there was none."""
         prev, self._prev = getattr(self, "_prev", None), None
         if prev is not None and not self._step_fitted():
             self._undo_host_step(prev[2])
-            self._step_once(*prev)
+            out = self._step_once(*prev)
             if not self._step_fitted():
                 raise RuntimeError("batched rasterizer: binning buffer overflowed twice in a row")
+            return out
+        return None
 
     def _undo_host_step(self, epoch):
         """Host-side bookkeeping of a step the device skipped (Adam step counts, lr schedule)."""

@@ -37,8 +37,9 @@ def gen_test_pose_subset():
                         trans=s["trans"].numpy()[idx], frame_index=idx, intrinsic=c["intrinsic"], extrinsic=c["extrinsic"])
 
 
-def gen_dataset_items():
-    """Items of the reference's own dataset classes (scene/dataset_mono.py) on the synthetic folder tests/dataset_fixture.py writes."""
+def _reference_dataset_items(stage2, every_item):
+    """Items of the reference's own dataset classes (scene/dataset_mono.py) on the synthetic folder tests/dataset_fixture.py writes:
+    the first and last item of each dataset, or every item."""
     import tempfile
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     from dataset_fixture import write_synthetic_dataset
@@ -48,13 +49,13 @@ def gen_dataset_items():
     fields = ("original_image", "world_view_transform", "projection_matrix", "full_proj_transform", "camera_center")
     out = {}
     with tempfile.TemporaryDirectory() as tmp:
-        mp = write_synthetic_dataset(tmp, stage2=True)
+        mp = write_synthetic_dataset(tmp, stage2=stage2)
         mp.no_mask = 1      # the reference's masked branch (dataset_mono.py:214) feeds an int8 array to PIL, which the Pillow of this image rejects
         sets = dict(train=ref.MonoDataset_train(mp, device="cpu"), test=ref.MonoDataset_test(mp, device="cpu"),
                     novel_pose=ref.MonoDataset_novel_pose(mp, device="cpu"))
         for name, dset in sets.items():
             out[f"{name}/len"] = np.array(len(dset))
-            for i in (0, len(dset) - 1):
+            for i in (range(len(dset)) if every_item else (0, len(dset) - 1)):
                 item = dset[i]
                 for k in fields:
                     if k in item:
@@ -63,7 +64,16 @@ def gen_dataset_items():
                 for k in ("pose_data", "transl_data", "inp_pos_map"):
                     if k in item:
                         out[f"{name}/{i}/{k}"] = np.asarray(item[k], dtype=np.float32)
-    np.savez_compressed(os.path.join(OUT, "dataset_items.npz"), **out)
+    return out
+
+
+def gen_dataset_items():
+    np.savez_compressed(os.path.join(OUT, "dataset_items.npz"), **_reference_dataset_items(stage2=True, every_item=False))
+
+
+def gen_dataset_items_stage1():
+    """Every item of the stage-1 datasets (no input position maps)."""
+    np.savez_compressed(os.path.join(OUT, "dataset_items_stage1.npz"), **_reference_dataset_items(stage2=False, every_item=True))
 
 
 def gen_smpl_A():
@@ -220,5 +230,6 @@ if __name__ == "__main__":
     gen_unet()
     gen_unet_full_size()
     gen_dataset_items()
+    gen_dataset_items_stage1()
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))

@@ -1,16 +1,16 @@
 """CPU: the reference's dataset folder contract (scene/dataset_mono.py) read by gaussianavatar_b200.dataset.  Pinned against the
-reference's OWN dataset classes run on the same synthetic folder: directly when /root/reference is importable (the build container),
-and through tests/golden/dataset_items.npz (written by oracle/gen_golden.py from those classes) everywhere."""
+reference's OWN dataset classes run on the same synthetic folder, through the items oracle/gen_golden.py stored from those classes:
+tests/golden/dataset_items.npz (first and last item of the stage-2 datasets) and tests/golden/dataset_items_stage1.npz (every item of
+the stage-1 datasets)."""
 import os
-import sys
 
 import numpy as np
-import pytest
 import torch
 
 from dataset_fixture import write_synthetic_dataset
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "dataset_items.npz")
+GOLD_STAGE1 = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "dataset_items_stage1.npz")
 FIELDS = ("original_image", "world_view_transform", "projection_matrix", "full_proj_transform", "camera_center")
 
 
@@ -43,25 +43,18 @@ def test_items_match_golden_from_reference_classes(tmp_path):
                 np.testing.assert_allclose(v, gold[f"{name}/{i}/{k}"], rtol=0, atol=1e-7, err_msg=f"{name}[{i}].{k}")
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/scene"), reason="reference not present (GPU box)")
 def test_items_match_reference_classes_directly(tmp_path):
+    """Every item of the stage-1 datasets, field for field, against what the reference's classes returned for the same folder."""
     mp, sets = _ours(tmp_path)
-    sys.path.insert(0, "/root/reference")
-    try:
-        from scene import dataset_mono as ref
-    finally:
-        sys.path.remove("/root/reference")
-    orig = ref.getProjectionMatrix       # numpy-1.x semantics of the reference's environment: np.float32 / python float -> float64 scalar
-    ref.getProjectionMatrix = lambda **kw: orig(**{**kw, "K": np.asarray(kw["K"]).astype(np.float64)})
-    refs = dict(train=ref.MonoDataset_train(mp, device="cpu"), test=ref.MonoDataset_test(mp, device="cpu"),
-                novel_pose=ref.MonoDataset_novel_pose(mp, device="cpu"))
+    gold = np.load(GOLD_STAGE1)
     for name, dset in sets.items():
-        assert len(dset) == len(refs[name])
+        assert len(dset) == int(gold[f"{name}/len"])
         for i in range(len(dset)):
-            a, b = _item_arrays(dset[i]), _item_arrays(refs[name][i])
-            assert a.keys() == b.keys()
+            a = _item_arrays(dset[i])
+            pfx = f"{name}/{i}/"
+            assert set(a) == {k[len(pfx):] for k in gold.files if k.startswith(pfx)}
             for k in a:
-                np.testing.assert_allclose(a[k], b[k], rtol=0, atol=1e-7, err_msg=f"{name}[{i}].{k}")
+                np.testing.assert_allclose(a[k], gold[pfx + k], rtol=0, atol=1e-7, err_msg=f"{name}[{i}].{k}")
 
 
 def test_device_decode_is_bit_identical_to_host_compositing(tmp_path):
